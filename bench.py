@@ -76,7 +76,13 @@ def parse():
     ap.add_argument("--matching", default="optimized", choices=["optimized", "advanced"])
     ap.add_argument("--cpu-sample-pairs", type=int, default=6)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the result records of the headline's last timed step to DIR/<field>.npy "
+                         "(float32 / float64), so that two builds can be compared output for output on the same inputs")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 arm")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -471,6 +477,20 @@ def parity_vs_oracle(gpu_results, cpu_results, what, gpu_T=lambda r: np.array(r.
                 tolerance="%g rad / %g m" % (ROT_TOL, TRANS_TOL))
 
 
+DUMP_FIELDS = ("T", "Tf", "pose_between", "final_hessian", "fitness", "converged", "valid", "iterations", "n_linearize", "n_error",
+               "lm_failed", "status")
+
+
+def dump_outputs(directory, jobs):
+    """One .npy per field of b200reg_result over every pair of `jobs` (lists of result records, in submission order): what
+    the caller of b200reg_batch_wait receives.  Integer and flag fields are stored as float64."""
+    recs = [r.as_dict() for job in jobs for r in job]
+    os.makedirs(directory, exist_ok=True)
+    for name in DUMP_FIELDS:
+        a = np.array([d[name] for d in recs])
+        np.save(os.path.join(directory, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
+
+
 def percentiles(x):
     x = np.asarray(x, np.float64)
     return dict(p50=float(np.percentile(x, 50)), p99=float(np.percentile(x, 99)), max=float(x.max()), n=int(len(x)))
@@ -570,6 +590,8 @@ def main():
     if batch_h is not batch:
         batch_h.close()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:  # the last timed step of the device-resident arm: 16 jobs x 16 pairs
+        dump_outputs(args.dump_outputs, res_dev[-JOBS_PER_STEP:])
 
     # one result per distinct pair (jobs 0..3 of the device arm), bit-identical across repeats and arms
     first = {(j + rank) % DISTINCT_JOBS: j for j in reversed(range(DISTINCT_JOBS))}  # sub-batch -> first job that ran it

@@ -66,6 +66,9 @@ def test_covariances_100k_match_oracle(ctx, ref_oracle, synth):
     assert np.median(err) < 1e-12 and np.quantile(err, 0.999) < 1e-6, (np.median(err), np.quantile(err, 0.999))
     gi, gd = ctx.knn(cl, dst[::7], 15)
     assert np.array_equal(gi, knn[::7]), "15-NN index lists must be bit-exact at 100k"
+    # the reference kd-tree's own lists on a seeded sample of these queries (tests/golden/make_golden.py ref_samples)
+    ref = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "knn_ref_nanoflann_100k.npz"))
+    assert np.array_equal(gi[ref["rows_self15"]], ref["idx_self15"]), "15-NN index lists must equal the reference kd-tree's"
     cl.destroy()
 
 
