@@ -6,10 +6,11 @@ from concurrent.futures import ThreadPoolExecutor
 PKG = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(PKG, "csrc")
 REPO = os.path.dirname(PKG)
-SOURCES = ["api.cu", "index_build.cu", "gicp.cu", "quatro.cu", "assemble.cu", "batch.cu"]
+SOURCES = ["api.cu", "index_build.cu", "gicp.cu", "quatro.cu", "assemble.cu", "batch.cu", "map.cu"]
 EXTRA = {"quatro.cu": ["-fmad=false"],    # fixed fp32 operation order for the FPFH / matcher arithmetic
-         "assemble.cu": ["-fmad=false"]}  # transformPcd / VoxelGrid / candidate distances as the (FMA-free) reference computes them
-HEADERS = ["internal.cuh", "knn.cuh", "smallmath.cuh", "fpfh_basis.cuh", os.path.join(REPO, "include", "b200reg.h")]
+         "assemble.cu": ["-fmad=false"],  # transformPcd / VoxelGrid / candidate distances as the (FMA-free) reference computes them
+         "map.cu": ["-fmad=false"]}       # the same transformPcd / VoxelGrid over the whole keyframe store
+HEADERS = ["internal.cuh", "voxel.cuh", "knn.cuh", "smallmath.cuh", "fpfh_basis.cuh", os.path.join(REPO, "include", "b200reg.h")]
 LIB = os.path.join(CSRC, "libb200reg.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-Xcompiler", "-fPIC",

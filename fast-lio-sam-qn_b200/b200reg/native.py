@@ -82,6 +82,7 @@ EXPORTS = [
     "b200reg_batch_wait", "b200reg_batch_wait_all", "b200reg_batch_launch_count", "b200reg_batch_depth",
     "b200reg_comm_unique_id", "b200reg_comm_init", "b200reg_comm_destroy", "b200reg_comm_rank", "b200reg_comm_world",
     "b200reg_allgather_results",
+    "b200reg_map_build", "b200reg_map_size", "b200reg_map_voxelized", "b200reg_map_get", "b200reg_map_destroy",
 ]
 
 
@@ -114,6 +115,7 @@ def lib():
         _lib.b200reg_batch_submit_icp.restype = C.c_int64
         _lib.b200reg_batch_submit_loop_closure.restype = C.c_int64
         _lib.b200reg_batch_launch_count.restype = C.c_int64
+        _lib.b200reg_map_size.restype = C.c_size_t
     return _lib
 
 
@@ -577,6 +579,21 @@ class Keyframes:
         if raw:
             return res, qi
         return [r.as_dict() for r in res], [x.as_dict() for x in qi]
+
+    def build_map(self, voxel_res=0.3, n_keyframes=0):
+        """The corrected global map (fast_lio_sam_qn.cpp:302-316, :398-411, :435-449): keyframes 0 .. n_keyframes-1 (0 = all)
+        transformed by their corrected poses, merged, voxelised at voxel_res.  -> (records (m, 4) float32 x y z intensity
+        in voxel-index order, voxelized); voxelized is False when PCL's int32 index guard tripped and the records are the
+        merged cloud unchanged."""
+        h = C.c_void_p()
+        _check(lib().b200reg_map_build(self.ctx.h, self.h, int(n_keyframes), C.c_double(voxel_res), C.byref(h)))
+        try:
+            out = np.empty((int(lib().b200reg_map_size(h)), 4), np.float32)
+            voxelized = bool(lib().b200reg_map_voxelized(h))
+            _check(lib().b200reg_map_get(self.ctx.h, h, out.ctypes.data_as(C.c_void_p)))
+        finally:
+            _check(lib().b200reg_map_destroy(self.ctx.h, h))
+        return out, voxelized
 
     def loop_factors(self, query_idx, closest_idx, raw_results):
         """The BetweenFactor records of a perform_loop_closure(..., raw=True) batch (fast_lio_sam_qn.cpp:220-237)."""

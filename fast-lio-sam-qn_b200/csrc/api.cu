@@ -42,6 +42,11 @@ void launch_ingest_world(const float* d_raw, int stride, int n, const double* d_
 void launch_pack_xyzi(const float* d_raw, int stride, int n, float4* d_out, cudaStream_t s);
 int launch_assemble_voxelize(const AssembleJob* d_jobs, const CloudDev* d_sort, int count, int max_total, const KeyframeDev* d_kfs,
                              const double* d_poses, float inv_leaf, cudaStream_t s);
+int launch_map_transform(const MapBlock* d_blocks, int nblocks, const double* d_poses, float inv_leaf, float4* d_merged,
+                         float* d_partials, MapInfo* d_info, cudaStream_t s);
+int launch_map_sort_heads(const float4* d_merged, int n, float inv_leaf, MapInfo* d_info, const CloudDev* d_sort, const CloudDev& sort,
+                          int key_bits, int* d_tile_cnt, int* d_tile_off, int* d_heads, float4* d_sorted, cudaStream_t s);
+int launch_map_centroids(const int* d_heads, const float4* d_sorted, int nv, float4* d_out, cudaStream_t s);
 }  // namespace b200
 
 using namespace b200;
@@ -1991,6 +1996,141 @@ int b200reg_perform_loop_closure(b200reg_ctx* c, b200reg_keyframes* kf, int coun
     b200reg_cloud_destroy(c, dc[k]);
   }
   return rc;
+}
+
+// ---- the corrected global map (map.cu) ----------------------------------------------------------------
+// The records get a cudaMalloc of their own: they outlive the call (the reason keyframe slabs do, §6b); the workspace
+// comes from the scratch pool.
+struct b200reg_map {
+  float4* d = nullptr;
+  size_t n = 0;
+  int voxelized = 0;
+};
+// the sort's look-back words carry 30-bit counts (index_build.cu: LB_MASK)
+constexpr size_t MAP_MAX_POINTS = ((size_t)1 << 30) - 1;
+
+int b200reg_map_build(b200reg_ctx* c, const b200reg_keyframes* kf, int n_keyframes, double voxel_res, b200reg_map** out) {
+  if (!c || !kf || !out) return fail(B200REG_EINVAL, "bad argument");
+  *out = nullptr;
+  const int nkall = (int)kf->pts.size();
+  if (nkall == 0) return fail(B200REG_EINVAL, "empty keyframe store");
+  if (n_keyframes < 0 || n_keyframes > nkall) return fail(B200REG_EINVAL, "n_keyframes out of range");
+  if (!(voxel_res > 0)) return fail(B200REG_EINVAL, "voxel_res must be positive");
+  const int nk = n_keyframes > 0 ? n_keyframes : nkall;
+  // block table: (keyframe, tile) -> source, first merged index, points
+  std::vector<MapBlock> blocks;
+  size_t total = 0;
+  for (int i = 0; i < nk; i++) {
+    for (int o = 0; o < kf->n[i]; o += MAP_TILE) blocks.push_back(MapBlock{kf->pts[i] + o, i, (int)(total + o), std::min(MAP_TILE, kf->n[i] - o), 0});
+    total += kf->n[i];
+    if (total > MAP_MAX_POINTS) return fail(B200REG_EINVAL, "more than 2^30 - 1 merged points");
+  }
+  const int n = (int)total, nb = (int)blocks.size();
+  const float inv_leaf = 1.0f / (float)voxel_res;
+  CU(cudaSetDevice(c->device));
+  cudaStream_t s = c->stream;
+  Scratch scratch(c);
+  float4* d_merged = nullptr;
+  float* d_partials = nullptr;
+  MapBlock* d_blocks = nullptr;
+  double* d_poses = nullptr;
+  MapInfo* d_info = nullptr;
+  CU(scratch.alloc((void**)&d_merged, (size_t)n * 16));
+  CU(scratch.alloc((void**)&d_partials, (size_t)nb * 24));
+  CU(scratch.alloc((void**)&d_blocks, sizeof(MapBlock) * (size_t)nb));
+  CU(scratch.alloc((void**)&d_poses, 128 * (size_t)nk));
+  CU(scratch.alloc((void**)&d_info, sizeof(MapInfo)));
+  CU(cudaMemcpyAsync(d_blocks, blocks.data(), sizeof(MapBlock) * (size_t)nb, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(d_poses, kf->poses.data(), 128 * (size_t)nk, cudaMemcpyHostToDevice, s));
+  MapInfo info;
+  {
+    ProfScope ps(c, CLS_MISC);
+    c->launches += launch_map_transform(d_blocks, nb, d_poses, inv_leaf, d_merged, d_partials, d_info, s);
+  }
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(&info, d_info, sizeof(MapInfo), cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  float4* rec = nullptr;
+  if (info.overflow) {  // PCL returns the merged cloud as it is
+    CU(cudaMalloc((void**)&rec, (size_t)n * 16));
+    const cudaError_t e = cudaMemcpyAsync(rec, d_merged, (size_t)n * 16, cudaMemcpyDeviceToDevice, s);
+    if (e != cudaSuccess) {
+      cudaFree(rec);
+      return fail(B200REG_ECUDA, std::string("map copy: ") + cudaGetErrorString(e));
+    }
+    c->prof_bytes[CLS_MISC] += 48.0 * n;  // 16 in + 16 merged + 16 copied
+    *out = new b200reg_map{rec, (size_t)n, 0};
+    return B200REG_OK;
+  }
+#ifndef B200REG_NO_SORT8
+  const int key_bits = info.key_bits <= 24 ? info.key_bits : 32;  // 3 x 8-bit digits, or the 3 x 11 bits of the sub-map grid
+#else  // development switch: every map on the 11-bit digits (profiles/map_build.py times the two against each other)
+  const int key_bits = 32;
+#endif
+  const int ntiles = (n + MAP_TILE - 1) / MAP_TILE;
+  const size_t ws = radix_sort_ws_bytes(n, key_bits);
+  CloudDev sd;
+  memset(&sd, 0, sizeof(sd));
+  sd.n = n;
+  int *d_tile_cnt = nullptr, *d_tile_off = nullptr, *d_heads = nullptr;
+  float4* d_sorted = nullptr;
+  CloudDev* d_sort = nullptr;
+  for (int b = 0; b < 2; b++) {
+    CU(scratch.alloc((void**)&sd.keys[b], (size_t)n * 4));
+    CU(scratch.alloc((void**)&sd.vals[b], (size_t)n * 4));
+  }
+  CU(scratch.alloc((void**)&sd.hist, ws));
+  CU(scratch.alloc((void**)&d_tile_cnt, (size_t)ntiles * 4));
+  CU(scratch.alloc((void**)&d_tile_off, (size_t)ntiles * 4));
+  CU(scratch.alloc((void**)&d_heads, ((size_t)n + 1) * 4));
+  CU(scratch.alloc((void**)&d_sorted, (size_t)n * 16));
+  CU(scratch.alloc((void**)&d_sort, sizeof(CloudDev)));
+  CU(cudaMemsetAsync(sd.hist, 0, ws, s));
+  CU(cudaMemcpyAsync(d_sort, &sd, sizeof(CloudDev), cudaMemcpyHostToDevice, s));
+  {
+    ProfScope ps(c, CLS_MISC);
+    c->launches += launch_map_sort_heads(d_merged, n, inv_leaf, d_info, d_sort, sd, key_bits, d_tile_cnt, d_tile_off, d_heads, d_sorted, s);
+  }
+  CU(cudaGetLastError());
+  int nv = 0;
+  CU(cudaMemcpyAsync(&nv, &d_info->voxels, 4, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  CU(cudaMalloc((void**)&rec, (size_t)nv * 16));
+  {
+    ProfScope ps(c, CLS_MISC);
+    c->launches += launch_map_centroids(d_heads, d_sorted, nv, rec, s);
+    c->prof_bytes[CLS_MISC] += 128.0 * n;  // 16 + 16 transform, 16 + 8 keys, 3 x 16 sort passes, 4 heads, 20 centroids
+  }
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    cudaFree(rec);
+    return fail(B200REG_ECUDA, std::string("map centroids: ") + cudaGetErrorString(e));
+  }
+  *out = new b200reg_map{rec, (size_t)nv, 1};
+  return B200REG_OK;
+}
+
+size_t b200reg_map_size(const b200reg_map* m) { return m ? m->n : 0; }
+
+int b200reg_map_voxelized(const b200reg_map* m) { return m ? m->voxelized : 0; }
+
+int b200reg_map_get(b200reg_ctx* c, const b200reg_map* m, float* xyzi_out) {
+  if (!c || !m || (!xyzi_out && m->n)) return fail(B200REG_EINVAL, "bad argument");
+  if (!m->n) return B200REG_OK;
+  CU(cudaSetDevice(c->device));
+  CU(cudaMemcpyAsync(xyzi_out, m->d, m->n * 16, cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return B200REG_OK;
+}
+
+int b200reg_map_destroy(b200reg_ctx* c, b200reg_map* m) {
+  if (!m) return B200REG_OK;
+  if (!c) return fail(B200REG_EINVAL, "ctx is NULL");
+  CU(cudaSetDevice(c->device));
+  CU(cudaStreamSynchronize(c->stream));  // nothing in flight may still write the records
+  CU(cudaFree(m->d));
+  delete m;
+  return B200REG_OK;
 }
 
 }  // extern "C"

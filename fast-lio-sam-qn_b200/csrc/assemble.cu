@@ -5,6 +5,7 @@
 // Keyframe clouds stay on the device from the moment they are added, so a loop-closure attempt moves no point data
 // over PCIe: candidate search, cloud assembly, voxel grid, index build and registration all start from HBM.
 #include "internal.cuh"
+#include "voxel.cuh"
 
 namespace b200 {
 
@@ -85,31 +86,25 @@ __global__ void __launch_bounds__(256) k_assemble(const AssembleJob* jobs, const
   }
 }
 
-// pcl::VoxelGrid first pass: idx = ijk0 + ijk1*dx + ijk2*dx*dy with ijk = floor(p * (1/L)) - float(min_b)
+// pcl::VoxelGrid first pass: the voxel index of every point (voxel.cuh)
 __global__ void __launch_bounds__(256) k_voxel_keys(const AssembleJob* jobs, float inv_leaf) {
   const AssembleJob& J = jobs[blockIdx.y];
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= J.total) return;
-  int min_b[3], div_b[3];
-  long long cells = 1;
+  float lo[3], hi[3];
 #pragma unroll
   for (int d = 0; d < 3; d++) {
-    const float lo = ord2f(J.bbox[d]), hi = ord2f(J.bbox[3 + d]);
-    min_b[d] = (int)floorf(lo * inv_leaf);
-    div_b[d] = (int)floorf(hi * inv_leaf) - min_b[d] + 1;
-    cells *= (long long)((hi - lo) * inv_leaf) + 1;
+    lo[d] = ord2f(J.bbox[d]);
+    hi[d] = ord2f(J.bbox[3 + d]);
   }
-  if (cells > 2147483647LL) {  // PCL: "Leaf size is too small ... Integer indices would overflow" -> input returned as is
+  const VoxelGridDev g = voxel_grid(lo, hi, inv_leaf);
+  if (voxel_grid_overflows(g)) {
     if (i == 0) J.counters[1] = 1;
     J.sort.keys[0][i] = (uint32_t)i;
     J.sort.vals[0][i] = (uint32_t)i;
     return;
   }
-  const float4 p = J.merged[i];
-  const int i0 = (int)(floorf(p.x * inv_leaf) - (float)min_b[0]);
-  const int i1 = (int)(floorf(p.y * inv_leaf) - (float)min_b[1]);
-  const int i2 = (int)(floorf(p.z * inv_leaf) - (float)min_b[2]);
-  J.sort.keys[0][i] = (uint32_t)(i0 + i1 * div_b[0] + i2 * div_b[0] * div_b[1]);
+  J.sort.keys[0][i] = voxel_key(J.merged[i], inv_leaf, g);
   J.sort.vals[0][i] = (uint32_t)i;
 }
 

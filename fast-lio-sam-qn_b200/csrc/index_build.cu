@@ -85,7 +85,13 @@ template <int BITS>
 __host__ __device__ inline size_t sort_ws_words(int n) {
   return (size_t)SORT_PASSES * (1 << BITS) + 32 + (size_t)SORT_PASSES * sort_tiles(n) * (1 << BITS);
 }
-size_t radix_sort_ws_bytes(int n, int key_bits) { return 4 * (key_bits <= 30 ? sort_ws_words<10>(n) : sort_ws_words<11>(n)); }
+// Keys of at most 24 bits (the global map's voxel indices, map.cu) take 3 passes of 8 bits: a look-back table of 256
+// instead of 2048 words per tile.
+constexpr int SORT8_MAX_BITS = 24;
+size_t radix_sort_ws_bytes(int n, int key_bits) {
+  if (key_bits <= SORT8_MAX_BITS) return 4 * sort_ws_words<8>(n);
+  return 4 * (key_bits <= 30 ? sort_ws_words<10>(n) : sort_ws_words<11>(n));
+}
 int radix_sort_result_buf(int) { return SORT_PASSES & 1; }
 
 // block-wide accumulation of the digit histograms of all passes (shared by the fused Morton kernel and k_sort_ghist)
@@ -309,11 +315,14 @@ __global__ void __launch_bounds__(SORT_THREADS) k_sort_pass(const CloudDev* clou
 
 // Stable LSD radix sort of (keys[0], vals[0]) of every descriptor; result in keys/vals[radix_sort_result_buf()].
 // Only the n / keys / vals / hist fields of the descriptors are used (also by the voxel grid, assemble.cu, and the
-// descriptor ordering, quatro.cu); hist must point to radix_sort_ws_bytes() ZEROED bytes.  key_bits <= 30: 3 x 10 bits,
-// otherwise 3 x 11 bits.
+// descriptor ordering, quatro.cu, and the global map, map.cu); hist must point to radix_sort_ws_bytes() ZEROED bytes.
+// key_bits <= 24: 3 x 8 bits, <= 30: 3 x 10 bits, otherwise 3 x 11 bits.
 int launch_radix_sort(const CloudDev* d_clouds, int count, int max_n, int key_bits, cudaStream_t s) {
   const dim3 grid(sort_tiles(max_n), count);
-  if (key_bits <= 30) {
+  if (key_bits <= SORT8_MAX_BITS) {
+    k_sort_ghist<8><<<grid, SORT_THREADS, SORT_PASSES * 256 * 4, s>>>(d_clouds);
+    for (int p = 0; p < SORT_PASSES; p++) k_sort_pass<8, false><<<grid, SORT_THREADS, 0, s>>>(d_clouds, p);
+  } else if (key_bits <= 30) {
     k_sort_ghist<10><<<grid, SORT_THREADS, SORT_PASSES * 1024 * 4, s>>>(d_clouds);
     for (int p = 0; p < SORT_PASSES; p++) k_sort_pass<10, false><<<grid, SORT_THREADS, 0, s>>>(d_clouds, p);
   } else {

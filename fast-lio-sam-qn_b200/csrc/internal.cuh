@@ -172,6 +172,29 @@ struct AssembleJob {  // one output cloud of setSrcAndDstCloud
   SortBufs sort;
 };
 
+// ---- global map: transformPcd over the whole store + one pcl::VoxelGrid (map.cu) ------------------
+constexpr int MAP_THREADS = 256;
+constexpr int MAP_TILE = 2048;  // points per block of the transform and of the run-head kernels
+struct MapBlock {               // one tile of one keyframe (built on the host: no per-point keyframe search)
+  const float4* src;            // first point of the tile in the keyframe's slab
+  int kf;                       // keyframe (row of the pose table)
+  int dst;                      // first merged index of the tile
+  int n;                        // points, <= MAP_TILE
+  int pad;
+};
+struct VoxelGridDev {
+  int min_b[3];     // floor(min * (1/L))
+  int div_b[3];     // floor(max * (1/L)) - min_b + 1
+  long long cells;  // PCL's overflow test: prod((int64)((max - min) * (1/L)) + 1)
+};
+struct MapInfo {    // written by the device, read back by the host between the phases of a map build
+  VoxelGridDev grid;
+  int overflow;     // PCL's int32 guard tripped: the map is the merged cloud
+  int key_bits;     // ceil(log2(div_b0 * div_b1 * div_b2)), at most 32
+  int voxels;       // occupied voxels
+  int pad;
+};
+
 // ---- Quatro matcher / solver workspace ---------------------------------------------------
 // per-pair device workspace of the matcher / solver
 struct MatchDev {

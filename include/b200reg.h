@@ -262,6 +262,19 @@ int b200reg_perform_loop_closure(b200reg_ctx* ctx, b200reg_keyframes* kf, int co
                                  const int32_t* closest_idx, const b200reg_loop_config* cfg, b200reg_result* out,
                                  b200reg_quatro_info* quatro_out);
 
+/* The corrected global map (fast_lio_sam_qn.cpp:302-316 /corrected_map, :398-411 <seq>_map.pcd, :435-449 result.pcd):
+ * every keyframe 0 .. n_keyframes-1 transformed by its CURRENT corrected pose (transformPcd: double math, float result,
+ * intensity carried), merged in keyframe order, then pcl::VoxelGrid at voxel_res (centroids of x, y, z, intensity in
+ * voxel-index order).  n_keyframes = 0: the whole store.  When PCL's int32 index guard trips (dx*dy*dz > INT32_MAX) the
+ * map is the merged cloud unchanged, as PCL returns it.  The records stay on the device until b200reg_map_destroy.
+ * B200REG_EINVAL: empty store, n_keyframes out of range, voxel_res <= 0, more than 2^30 - 1 merged points.            */
+typedef struct b200reg_map b200reg_map;
+int b200reg_map_build(b200reg_ctx* ctx, const b200reg_keyframes* kf, int n_keyframes, double voxel_res, b200reg_map** out);
+size_t b200reg_map_size(const b200reg_map* map);       /* records (x, y, z, intensity)                                 */
+int b200reg_map_voxelized(const b200reg_map* map);     /* 1: voxelised; 0: PCL's int32 guard tripped, records = merged */
+int b200reg_map_get(b200reg_ctx* ctx, const b200reg_map* map, float* xyzi_out);  /* size x 4 floats, voxel-index order */
+int b200reg_map_destroy(b200reg_ctx* ctx, b200reg_map* map);
+
 /* Result consumption (SURVEY.md §8f rank 3; fast_lio_sam_qn/src/fast_lio_sam_qn.cpp:220-237): the loop constraint the
  * reference hands to GTSAM for an accepted registration,
  *   BetweenFactor<Pose3>(latest.idx_, closest_idx, pose_from.between(pose_to), Diagonal::Variances(score x 6)),
